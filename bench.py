@@ -67,7 +67,31 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--updates-per-launch", type=int, default=20)
     ap.add_argument("--exchange", default="auto", choices=["auto", "nccl", "p2p"], help="N > 1: how the [obs | reward | done] rows reach the other ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (observation / reward / done rows, flags, and the goal, AMP "
+                         "observation and imitation reward of the AMP scenes) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared")
     return ap.parse_args()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, gathered, local, num_envs):
+    """gathered: name -> array [world, N, ...]; local: name -> array [N, ...] (this rank's environments).  Written as float32 .npy files.
+    Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of the environments is kept (the same ids in every array, listed in env_ids.npy)."""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in list(gathered.items()) + list(local.items())}
+    per_env = sum(v.nbytes for v in arrays.values()) / num_envs
+    keep = None
+    if per_env * num_envs > DUMP_LIMIT_BYTES:
+        n = max(1, int((DUMP_LIMIT_BYTES - 8 * num_envs) // per_env))
+        keep = np.sort(np.random.default_rng(0).choice(num_envs, size=n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        if keep is not None:
+            v = v[:, keep] if k in gathered else v[keep]
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    if keep is not None:
+        np.save(os.path.join(out_dir, "env_ids.npy"), keep.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------- CPU arm (oracle = port of the reference path)
@@ -296,6 +320,16 @@ def main():
         torch.cuda.synchronize()
         sampler.stop_flag = True; sampler.join(timeout=2)
         launches = core.counters()[0] - l0 + a.steps * xchg.launches_per_step
+        if a.dump_outputs and rank == 0:
+            obs, rew, done = xchg.rows(a.preroll + a.warmup + a.steps - 1)
+            local = {"flags": flags}
+            if amp:
+                local.update(amp_obs_agent=amp_buf, reward_imitate=rim_buf)
+                if core.dims.goal_size:
+                    local["goal"] = goal_buf
+            stream.synchronize()
+            dump_outputs(a.dump_outputs, {k: v.cpu().numpy() for k, v in (("obs", obs), ("reward", rew), ("done", done))},
+                         {k: v.cpu().numpy() for k, v in local.items()}, N)
         per_step = np.array([x.elapsed_time(y) for x, y in step_ms])
         per_kern = np.array([x.elapsed_time(y) for x, y in upd_ms]) / (20 // upl)
         total_ms = float(per_step.sum())

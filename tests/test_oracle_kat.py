@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+from deepmimic_b200.assets import reference_root
 from tests.oracle_binding import Oracle
 
 SPINKICK = ["--arg_file", "args/run_humanoid3d_spinkick_args.txt"]
@@ -374,8 +375,12 @@ def _run_policy_in_oracle(o, actor, t0, steps=600):
     return len(rew), float(np.mean(rew)), o.has_fallen(), o.get_time()
 
 
-def _fixture_actor():
-    f = np.load(os.path.join(os.path.dirname(__file__), "golden", "policy_humanoid3d_spinkick_fp16.npz"))
+def _fixture_path(char, clip):
+    return os.path.join(os.path.dirname(__file__), "golden", "policy_%s_%s_fp16.npz" % (char, clip))
+
+
+def _fixture_actor(char="humanoid3d", clip="spinkick"):
+    f = np.load(_fixture_path(char, clip))
     g = lambda k: f[k].astype(np.float64)
     return dict(hidden=[(g("w0"), g("b0")), (g("w1"), g("b1"))], mean=(g("wm"), g("bm")), s_norm_mean=g("s_mean"), s_norm_std=g("s_std"),
                 a_norm_mean=g("a_mean"), a_norm_std=g("a_std"))
@@ -396,17 +401,21 @@ def test_pretrained_reference_policy_tracks_the_clip_in_the_oracle(asset_root):
 @pytest.mark.parametrize("char,clip,min_reward", [("humanoid3d", "walk", 0.8), ("humanoid3d", "backflip", 0.75), ("humanoid3d", "cartwheel", 0.8),
                                                    ("humanoid3d", "jump", 0.85), ("dog3d", "trot", 0.85), ("dog3d", "pace", 0.8), ("dog3d", "canter", 0.8),
                                                    ("dog3d", "spin", 0.75)])   # spin: --sync_char_root_rot true (0.44 when the sync only touched the pose, 0.80 with RotateOrigin)
-def test_more_pretrained_policies_from_the_reference_tree(char, clip, min_reward):
-    """Same check for other skills, reading the TF1 checkpoints directly (deepmimic_b200/tf_checkpoint.py); needs the reference checkout."""
-    ref = "/root/reference"
-    ckpt = os.path.join(ref, "data/policies/%s/%s_%s.ckpt" % (char, char, clip))
-    if not os.path.exists(ckpt + ".index"):
-        pytest.skip("reference checkout with pretrained policies not available")
-    from deepmimic_b200.tf_checkpoint import load_actor
-    a = load_actor(ckpt)
-    a = {k: ([(w.astype(np.float64), b.astype(np.float64)) for w, b in v] if k == "hidden" else (tuple(x.astype(np.float64) for x in v) if k == "mean" else v.astype(np.float64)))
-         for k, v in a.items()}
-    o = Oracle(["--arg_file", "args/run_%s_%s_args.txt" % (char, clip)], ref)
+def test_more_pretrained_policies_from_the_reference_tree(asset_root, char, clip, min_reward):
+    """Same check for other skills: the committed fp16 fixture of the skill's policy on the committed assets where there is one (dog3d trot),
+    else the TF1 checkpoint read directly (deepmimic_b200/tf_checkpoint.py) from a reference checkout."""
+    if os.path.exists(_fixture_path(char, clip)):
+        a, root = _fixture_actor(char, clip), asset_root
+    else:
+        root = reference_root()
+        ckpt = os.path.join(root or "", "data/policies/%s/%s_%s.ckpt" % (char, char, clip))
+        if not root or not os.path.exists(ckpt + ".index"):
+            pytest.skip("reference checkout with pretrained policies not available (set DEEPMIMIC_REFERENCE_ROOT)")
+        from deepmimic_b200.tf_checkpoint import load_actor
+        a = load_actor(ckpt)
+        a = {k: ([(w.astype(np.float64), b.astype(np.float64)) for w, b in v] if k == "hidden" else (tuple(x.astype(np.float64) for x in v) if k == "mean" else v.astype(np.float64)))
+             for k, v in a.items()}
+    o = Oracle(["--arg_file", "args/run_%s_%s_args.txt" % (char, clip)], root)
     o.L.dmo_set_mode(o.h, 1)
     n, mean_r, fallen, t = _run_policy_in_oracle(o, a, 0.0)
     assert n == 600 and not fallen, (clip, n, fallen)
@@ -418,10 +427,10 @@ def test_more_pretrained_policies_from_the_reference_tree(char, clip, min_reward
 def test_pretrained_amp_policies_stay_up_in_the_oracle(arg_file, ckpt):
     """The reference's AMP policies (scene imitate_amp: no phase input, state 226 / 346) are not phase-locked to the clip, so the imitation
     reward says little -- but they must keep the character going (back-flipping, crawling, trotting) for the whole 20 s without a fall."""
-    ref = "/root/reference"
-    path = os.path.join(ref, "data/policies", ckpt + ".ckpt")
-    if not os.path.exists(path + ".index"):
-        pytest.skip("reference checkout with pretrained policies not available")
+    ref = reference_root()
+    path = os.path.join(ref or "", "data/policies", ckpt + ".ckpt")
+    if not ref or not os.path.exists(path + ".index"):
+        pytest.skip("reference checkout with pretrained policies not available (set DEEPMIMIC_REFERENCE_ROOT)")
     from deepmimic_b200.tf_checkpoint import load_actor
     a = load_actor(path)
     a = {k: ([(w.astype(np.float64), b.astype(np.float64)) for w, b in v] if k == "hidden" else (tuple(x.astype(np.float64) for x in v) if k == "mean" else v.astype(np.float64)))

@@ -94,9 +94,11 @@ def test_gated_policy_matches_numpy_restatement_of_the_reference_net():
 
 def test_checkpoint_reader_returns_the_gate_layers_of_a_task_policy():
     import os
-    ckpt = "/root/reference/data/policies/humanoid3d_amp/humanoid3d_amp_heading_locomotion.ckpt"
-    if not os.path.exists(ckpt + ".index"):
-        pytest.skip("reference checkout with pretrained policies not available")
+    from deepmimic_b200.assets import reference_root
+    ref = reference_root()
+    ckpt = os.path.join(ref or "", "data/policies/humanoid3d_amp/humanoid3d_amp_heading_locomotion.ckpt")
+    if not ref or not os.path.exists(ckpt + ".index"):
+        pytest.skip("reference checkout with pretrained policies not available (set DEEPMIMIC_REFERENCE_ROOT)")
     from deepmimic_b200.tf_checkpoint import load_actor
     a = load_actor(ckpt)
     assert [w.shape for w, _ in a["hidden"]] == [(229, 1024), (1024, 512)] and a["gate_common"][0].shape == (3, 128)

@@ -10,6 +10,7 @@ import os
 import numpy as np
 import pytest
 
+from deepmimic_b200.assets import reference_root
 from tests.oracle_binding import Oracle
 
 MINI = ["--motion_file", "data/datasets/test_clips_mini.txt"]
@@ -261,11 +262,14 @@ def gated_actor_mode(actor, s, g):
     return (h @ actor["mean"][0] + actor["mean"][1]) * actor["a_norm_std"] + actor["a_norm_mean"]
 
 
-def run_task_policy(arg_file, ckpt, seed, clip, t0, theta, steps=600):
-    from deepmimic_b200.tf_checkpoint import load_actor
-    ref = "/root/reference"
-    a = _f64(load_actor(os.path.join(ref, "data/policies", ckpt + ".ckpt")))
-    o = Oracle(["--arg_file", arg_file], ref)
+# the committed archive's 56-entry clip dataset (the reference's locomotion dataset has 56 clips but is not in the archive): the reset
+# clip ids of the policy pins below exist in it, and its clips are the archive's walk / run clips
+SYNTH56 = ["--motion_file", "data/datasets/synthetic_locomotion_56.txt"]
+
+
+def run_task_policy(asset_root, task, arg_file, seed, clip, t0, theta, steps=600):
+    a = fixture_task_actor(task)
+    o = Oracle(SYNTH56 + ["--arg_file", arg_file], asset_root)
     o.L.dmo_set_mode(o.h, 1)
     o.set_task_stream(seed, 0, 0)
     o.reset(t0, theta, 20.0, clip=clip)
@@ -285,28 +289,24 @@ def run_task_policy(arg_file, ckpt, seed, clip, t0, theta, steps=600):
     return len(rew), float(np.mean(rew)), o.has_fallen(), succ, np.array(dist), o
 
 
-needs_reference = pytest.mark.skipif(not os.path.exists("/root/reference/data/policies/humanoid3d_amp/humanoid3d_amp_target_locomotion.ckpt.index"),
-                                     reason="reference checkout with pretrained policies not available")
+needs_reference = pytest.mark.skipif(not (reference_root() and os.path.exists(os.path.join(reference_root(), "data/policies/humanoid3d_amp/humanoid3d_amp_strike_walk_punch.ckpt.index"))),
+                                     reason="reference checkout with pretrained policies not available (set DEEPMIMIC_REFERENCE_ROOT)")
 
 
-@needs_reference
 @pytest.mark.parametrize("seed,clip,t0,theta", [(1, 0, 0.3, 0.4), (2, 30, 1.0, -2.5)])
-def test_pretrained_target_policy_walks_to_its_targets_in_the_oracle(seed, clip, t0, theta):
-    """The reference's own target-location policy (trained in the real simulator on goals from the real RecordGoal) reaches the targets
-    the oracle draws: it spends a good part of the 20 s inside the 0.5 m success radius and never falls.  A wrong goal frame, sign or
+def test_pretrained_target_policy_walks_to_its_targets_in_the_oracle(asset_root, seed, clip, t0, theta):
+    """The reference's own target-location policy (fp16 fixture; trained in the real simulator on goals from the real RecordGoal) reaches the
+    targets the oracle draws: it spends a good part of the 20 s inside the 0.5 m success radius and never falls.  A wrong goal frame, sign or
     target update would send it elsewhere."""
-    n, mean_r, fallen, succ, dist, o = run_task_policy("args/run_amp_target_humanoid3d_locomotion_args.txt", "humanoid3d_amp/humanoid3d_amp_target_locomotion",
-                                                       seed, clip, t0, theta)
+    n, mean_r, fallen, succ, dist, o = run_task_policy(asset_root, "target", "args/train_amp_target_humanoid3d_locomotion_args.txt", seed, clip, t0, theta)
     assert n == 600 and not fallen, (n, fallen)
     assert succ >= 60 and dist.min() < 0.2 and mean_r > 0.4, (succ, dist.min(), mean_r)
 
 
-@needs_reference
 @pytest.mark.parametrize("seed,clip,t0,theta", [(1, 0, 0.3, 0.4), (5, 17, 0.5, 2.0)])
-def test_pretrained_heading_policy_follows_heading_and_speed_in_the_oracle(seed, clip, t0, theta):
+def test_pretrained_heading_policy_follows_heading_and_speed_in_the_oracle(asset_root, seed, clip, t0, theta):
     """Same for the heading policy: the task reward exp(-0.25 (v* - v)^2) of the oracle's heading / speed commands stays high for 20 s."""
-    n, mean_r, fallen, succ, dist, o = run_task_policy("args/run_amp_heading_humanoid3d_locomotion_args.txt", "humanoid3d_amp/humanoid3d_amp_heading_locomotion",
-                                                       seed, clip, t0, theta)
+    n, mean_r, fallen, succ, dist, o = run_task_policy(asset_root, "heading", "args/train_amp_heading_humanoid3d_locomotion_args.txt", seed, clip, t0, theta)
     assert n == 600 and not fallen, (n, fallen)
     assert mean_r > 0.8, mean_r
 
@@ -618,15 +618,13 @@ def test_getup_recovery_episodes_and_test_mode_getups(asset_root):
     assert began
 
 
-@needs_reference
 @pytest.mark.parametrize("clip", [2, 3])
-def test_pretrained_getup_policy_stands_up_and_follows_the_heading_in_the_oracle(clip):
-    """The reference's heading + get-up policy starts lying on the ground (get-up clips 2 / 3 of its dataset), stands up (head above 1.3 m)
-    and then earns the heading reward for the rest of the 20 s (0.97 measured over the last 10 s)."""
-    from deepmimic_b200.tf_checkpoint import load_actor
-    ref = "/root/reference"
-    a = _f64(load_actor(os.path.join(ref, "data/policies/humanoid3d_amp/humanoid3d_amp_heading_getup_locomotion_getup.ckpt")))
-    o = Oracle(["--arg_file", "args/run_amp_heading_getup_humanoid3d_locomotion_getup_args.txt"], ref)
+def test_pretrained_getup_policy_stands_up_and_follows_the_heading_in_the_oracle(asset_root, clip):
+    """The reference's heading + get-up policy (fp16 fixture) starts lying on the ground (get-up clips 2 / 3 of its dataset, which the
+    committed archive holds in full), stands up (head above 1.3 m) and then earns the heading reward for the rest of the 20 s (0.97 measured
+    over the last 10 s)."""
+    a = fixture_task_actor("heading_getup")
+    o = Oracle(["--arg_file", "args/train_amp_heading_getup_humanoid3d_locomotion_getup_args.txt"], asset_root)
     o.L.dmo_set_mode(o.h, 1)
     o.set_task_stream(4, 0, 0)
     o.reset(0.0, 0.4, 20.0, clip=clip)
@@ -721,7 +719,7 @@ def test_pretrained_strike_policy_punches_the_target_in_the_oracle(seed, far):
     """The reference's walk-and-punch policy hits the oracle-drawn target with its hand (fast enough, from the right side) and holds for the 2 s
     that make the episode a success (terminate code 2) -- also when it first has to walk 5 m to get there."""
     from deepmimic_b200.tf_checkpoint import load_actor
-    ref = "/root/reference"
+    ref = reference_root()
     a = _f64(load_actor(os.path.join(ref, "data/policies/humanoid3d_amp/humanoid3d_amp_strike_walk_punch.ckpt")))
     o = Oracle(["--arg_file", "args/run_amp_strike_humanoid3d_walk_punch_args.txt"], ref)
     o.L.dmo_set_mode(o.h, 1)

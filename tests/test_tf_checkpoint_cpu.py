@@ -1,6 +1,7 @@
 """Hermetic test of deepmimic_b200/tf_checkpoint.py: a TensorBundle checkpoint (LevelDB-format .index table + .data shard) is written here
 byte by byte in the layout tf.train.Saver produces (prefix-compressed keys, restart array, block trailer, index block, 48-byte footer with
-the table magic; BundleEntryProto values) and read back.  The tests against the reference's real checkpoints need /root/reference."""
+the table magic; BundleEntryProto values) and read back.  The tests against the reference's real checkpoints need a reference checkout
+($DEEPMIMIC_REFERENCE_ROOT)."""
 import os
 import struct
 
@@ -97,6 +98,33 @@ def test_reads_back_a_hand_written_tensor_bundle(tmp_path):
     act = load_actor(prefix)
     assert [w.shape for w, _ in act["hidden"]] == [(7, 5), (5, 4)] and act["mean"][0].shape == (4, 3) and "gate_common" not in act
     assert np.array_equal(act["s_norm_std"], tensors["agent/resource/s_norm/std"]) and "g_norm_mean" not in act
+
+
+def test_reads_the_gate_layers_of_a_task_policy_bundle(tmp_path):
+    """fc_2layers_gated_1024units layout (gate_common, per hidden layer gate<i>/0/dense -> gate<i>/dense bias head, gate<i>/dense_1 scale head)
+    written with the tensors of the committed heading-policy fixture: load_actor returns the gate layers with the shapes of the reference's
+    humanoid3d_amp_heading_locomotion checkpoint and the fixture's values."""
+    f = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "policy_humanoid3d_amp_heading_locomotion_fp16.npz"))
+    g = lambda k: f[k].astype(np.float32)
+    a, r = "agent/main/actor/", "agent/resource/"
+    tensors = {a + "0/dense/kernel": g("w0"), a + "0/dense/bias": g("b0"), a + "1/dense/kernel": g("w1"), a + "1/dense/bias": g("b1"),
+               a + "dist_gauss_diag/mean/kernel": g("wm"), a + "dist_gauss_diag/mean/bias": g("bm"), a + "dist_gauss_diag/logstd/bias": g("logstd"),
+               a + "gate_common/0/dense/kernel": g("gcw"), a + "gate_common/0/dense/bias": g("gcb")}
+    for i in range(2):
+        for head, key in (("0/dense", "hidden"), ("dense", "bias"), ("dense_1", "scale")):
+            tensors[a + "gate%d/%s/kernel" % (i, head)] = g("g%d_%s_w" % (i, key))
+            tensors[a + "gate%d/%s/bias" % (i, head)] = g("g%d_%s_b" % (i, key))
+    for nm, key in (("s_norm", "s"), ("g_norm", "g"), ("a_norm", "a")):
+        tensors[r + nm + "/mean"], tensors[r + nm + "/std"] = g(key + "_mean"), g(key + "_std")
+    prefix = str(tmp_path / "model.ckpt")
+    write_bundle(prefix, tensors)
+    act = load_actor(prefix)
+    assert [w.shape for w, _ in act["hidden"]] == [(229, 1024), (1024, 512)] and act["gate_common"][0].shape == (3, 128)
+    assert [gt["scale"][0].shape for gt in act["gates"]] == [(64, 1024), (64, 512)] and act["g_norm_mean"].shape == (3,)
+    for i in range(2):
+        for key in ("hidden", "bias", "scale"):
+            assert np.array_equal(act["gates"][i][key][0], g("g%d_%s_w" % (i, key))) and np.array_equal(act["gates"][i][key][1], g("g%d_%s_b" % (i, key)))
+    assert np.array_equal(act["gate_common"][0], g("gcw")) and np.array_equal(act["g_norm_std"], g("g_std"))
 
 
 def test_rejects_files_that_are_not_tensor_bundles(tmp_path):
