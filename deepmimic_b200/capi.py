@@ -99,21 +99,18 @@ def _dptr(a):
     return a.ctypes.data_as(C.POINTER(C.c_double)) if a is not None else None
 
 
-class BatchedCore:
-    """Thin object wrapper over a dm_handle."""
+class _Handle:
+    """What a device handle (dm_create) and a host-only handle (dm_load_host) share: the host model's tables, the launch plan, close()."""
+    h = None
 
-    def __init__(self, args, num_envs, asset_root, device=0, seed=0, global_env_offset=0):
-        L = lib()
+    def _open(self, create, args, asset_root, *extra):
         enc = [a.encode() for a in args]
-        arr = (C.c_char_p * len(enc))(*enc)
-        self.h = L.dm_create(asset_root.encode(), len(enc), arr, num_envs, device, seed, global_env_offset)
-        if not self.h:
-            raise RuntimeError("dm_create failed: %s" % L.dm_last_error().decode())
-        self.h = C.c_void_p(self.h)
-        d = DmDims()
-        L.dm_get_dims(self.h, C.byref(d))
-        self.dims = d
-        self.num_envs = d.num_envs
+        h = create(asset_root.encode(), len(enc), (C.c_char_p * len(enc))(*enc), *extra)
+        if not h:
+            raise RuntimeError("%s failed: %s" % (create.__name__, lib().dm_last_error().decode()))
+        self.h = C.c_void_p(h)
+        self.dims = DmDims()
+        self._chk(lib().dm_get_dims(self.h, C.byref(self.dims)))
 
     def _chk(self, rc):
         if rc != 0:
@@ -136,6 +133,42 @@ class BatchedCore:
         self._chk(lib().dm_get_static(self.h, kind, _dptr(out)))
         return out
 
+    def plan_launch(self, num_envs, smem_bytes_per_block=232448, num_sms=148):
+        """dm_plan_launch: launch plan of the step kernel on a device with that much opt-in shared memory per block and that many SMs (B200 defaults)"""
+        out = (C.c_int * 9)()
+        self._chk(lib().dm_plan_launch(self.h, int(num_envs), int(smem_bytes_per_block), int(num_sms), out))
+        keys = ("tile_width", "envs_per_block", "blocks", "smem_bytes", "max_rows", "env_floats", "hot_floats", "y_offset", "padded_envs")
+        return dict(zip(keys, [int(v) for v in out]))
+
+    def task_params(self):
+        out = np.zeros(48, dtype=np.float64)     # [0:16] dm_task.cuh constants, [16:48] dm_task_ext.cuh constants
+        key = (C.c_uint64 * 2)()
+        self._chk(lib().dm_get_task_params(self.h, _dptr(out), key))
+        return out, int(key[0]), int(key[1])
+
+    def clip_table(self):
+        n = C.c_int(0)
+        self._chk(lib().dm_get_clip_table(self.h, C.byref(n), None, None))
+        dur, cdf = np.zeros(n.value), np.zeros(n.value)
+        self._chk(lib().dm_get_clip_table(self.h, C.byref(n), _dptr(dur), _dptr(cdf)))
+        return dur, cdf
+
+    def set_sample_count(self, count):
+        self._chk(lib().dm_set_sample_count(self.h, int(count)))
+
+    def time_limits(self):
+        out = np.zeros(3, dtype=np.float64)
+        self._chk(lib().dm_get_time_limits(self.h, _dptr(out)))
+        return out
+
+
+class BatchedCore(_Handle):
+    """Thin object wrapper over a dm_handle."""
+
+    def __init__(self, args, num_envs, asset_root, device=0, seed=0, global_env_offset=0):
+        self._open(lib().dm_create, args, asset_root, num_envs, device, seed, global_env_offset)
+        self.num_envs = self.dims.num_envs
+
     def scene_name(self):
         buf = C.create_string_buffer(64)
         self._chk(lib().dm_get_scene_name(self.h, buf, 64))
@@ -149,13 +182,6 @@ class BatchedCore:
         else:   # task scenes with a clip dataset: the controller's clip draw injected
             c = np.ascontiguousarray(clip, dtype=np.int32)
             self._chk(lib().dm_reset_clips(self.h, 1 if force_all else 0, c.ctypes.data_as(C.POINTER(C.c_int)), _dptr(kt), _dptr(mt), _dptr(th)))
-
-    def clip_table(self):
-        n = C.c_int(0)
-        lib().dm_get_clip_table(self.h, C.byref(n), None, None)
-        dur, cdf = np.zeros(n.value), np.zeros(n.value)
-        lib().dm_get_clip_table(self.h, C.byref(n), _dptr(dur), _dptr(cdf))
-        return dur, cdf
 
     def set_action(self, actions):  # torch float32 cuda tensor [N, A]
         self._chk(lib().dm_set_action(self.h, C.c_void_p(actions.data_ptr())))
@@ -187,20 +213,6 @@ class BatchedCore:
         b = np.ascontiguousarray(block, dtype=np.float64)
         self._chk(lib().dm_set_task_state(self.h, env, _dptr(b)))
 
-    def plan_launch(self, num_envs, smem_bytes_per_block=232448, num_sms=148):
-        """dm_plan_launch: launch plan of the step kernel on a device with that much opt-in shared memory per block and that many SMs (B200 defaults)"""
-        out = (C.c_int * 9)()
-        if lib().dm_plan_launch(self.h, int(num_envs), int(smem_bytes_per_block), int(num_sms), out) != 0:
-            raise RuntimeError(lib().dm_last_error().decode())
-        keys = ("tile_width", "envs_per_block", "blocks", "smem_bytes", "max_rows", "env_floats", "hot_floats", "y_offset", "padded_envs")
-        return dict(zip(keys, [int(v) for v in out]))
-
-    def task_params(self):
-        out = np.zeros(48, dtype=np.float64)     # [0:16] dm_task.cuh constants, [16:48] dm_task_ext.cuh constants
-        key = (C.c_uint64 * 2)()
-        self._chk(lib().dm_get_task_params(self.h, _dptr(out), key))
-        return out, int(key[0]), int(key[1])
-
     def amp_obs_agent(self, out):  # torch float32 cuda tensor [N, amp_obs_size]
         self._chk(lib().dm_record_amp_obs_agent(self.h, C.c_void_p(out.data_ptr())))
 
@@ -220,14 +232,6 @@ class BatchedCore:
 
     def set_mode(self, mode):
         self._chk(lib().dm_set_mode(self.h, mode))
-
-    def set_sample_count(self, count):
-        self._chk(lib().dm_set_sample_count(self.h, int(count)))
-
-    def time_limits(self):
-        out = np.zeros(3, dtype=np.float64)
-        self._chk(lib().dm_get_time_limits(self.h, _dptr(out)))
-        return out
 
     def step_host(self, actions, dt, n_updates, state, reward, flags, reset_done=False):  # numpy host arrays
         p = lambda a: None if a is None else C.c_void_p(a.ctypes.data)
@@ -297,85 +301,28 @@ class BatchedCore:
         return lib().dm_stream(self.h)
 
 
-class HostModel:
+class HostModel(_Handle):
     """dm_load_host handle: the host loaders and the flat model, no device (used by the CPU tests and by tools)."""
     INFO = dict(parents=0, joint_types=1, dof_offsets=2, pose_offsets=3, fall_bodies=4, end_effectors=5)
 
     def __init__(self, args, asset_root):
-        L = lib()
-        enc = [a.encode() for a in args]
-        arr = (C.c_char_p * len(enc))(*enc)
-        h = L.dm_load_host(asset_root.encode(), len(enc), arr)
-        if not h:
-            raise RuntimeError("dm_load_host failed: %s" % L.dm_last_error().decode())
-        self.h = C.c_void_p(h)
-        self.dims = DmDims()
-        L.dm_get_dims(self.h, C.byref(self.dims))
-
-    def static(self, kind):
-        n = self.dims.state_size if kind in (DM_STATE_OFFSET, DM_STATE_SCALE, DM_STATE_NORM_GROUPS) else self.dims.action_size
-        out = np.zeros(n, dtype=np.float64)
-        if lib().dm_get_static(self.h, kind, _dptr(out)) != 0:
-            raise RuntimeError(lib().dm_last_error().decode())
-        return out
-
-    def plan_launch(self, num_envs, smem_bytes_per_block=232448, num_sms=148):
-        """dm_plan_launch: launch plan of the step kernel on a device with that much opt-in shared memory per block and that many SMs (B200 defaults)"""
-        out = (C.c_int * 9)()
-        if lib().dm_plan_launch(self.h, int(num_envs), int(smem_bytes_per_block), int(num_sms), out) != 0:
-            raise RuntimeError(lib().dm_last_error().decode())
-        keys = ("tile_width", "envs_per_block", "blocks", "smem_bytes", "max_rows", "env_floats", "hot_floats", "y_offset", "padded_envs")
-        return dict(zip(keys, [int(v) for v in out]))
-
-    def task_params(self):
-        out = np.zeros(48, dtype=np.float64)     # [0:16] dm_task.cuh constants, [16:48] dm_task_ext.cuh constants
-        key = (C.c_uint64 * 2)()
-        lib().dm_get_task_params(self.h, _dptr(out), key)
-        return out, int(key[0]), int(key[1])
-
-    def clip_table(self):
-        n = C.c_int(0)
-        lib().dm_get_clip_table(self.h, C.byref(n), None, None)
-        dur, cdf = np.zeros(n.value), np.zeros(n.value)
-        lib().dm_get_clip_table(self.h, C.byref(n), _dptr(dur), _dptr(cdf))
-        return dur, cdf
-
-    def set_sample_count(self, count):
-        if lib().dm_set_sample_count(self.h, int(count)) != 0:
-            raise RuntimeError(lib().dm_last_error().decode())
-
-    def time_limits(self):
-        out = np.zeros(3, dtype=np.float64)
-        lib().dm_get_time_limits(self.h, _dptr(out))
-        return out
+        self._open(lib().dm_load_host, args, asset_root)
 
     def info(self, name):
         out = (C.c_int * self.dims.num_joints)()
-        if lib().dm_get_model_info(self.h, self.INFO[name], out) != 0:
-            raise RuntimeError(lib().dm_last_error().decode())
+        self._chk(lib().dm_get_model_info(self.h, self.INFO[name], out))
         return np.array(out[:], dtype=np.int64)
 
     def link_table(self):
         """[num_joints, 24]: mass, inertiaB[3], inertiaD[3], dvec[3], evec[3], zrot xyzw, axis[3], half extents[3], breaking threshold"""
         out = np.zeros((self.dims.num_joints, 24), dtype=np.float64)
-        lib().dm_get_link_table(self.h, _dptr(out))
+        self._chk(lib().dm_get_link_table(self.h, _dptr(out)))
         return out
 
     def layout(self):
         out = (C.c_int * 6)()
-        lib().dm_get_model_info(self.h, 6, out)
+        self._chk(lib().dm_get_model_info(self.h, 6, out))
         return dict(zip(("links", "dofs", "chain_stride", "tree_depth", "frames", "loop"), out[:]))
-
-    def close(self):
-        if self.h:
-            lib().dm_destroy(self.h)
-            self.h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
 
 class TensorCoreMLP:

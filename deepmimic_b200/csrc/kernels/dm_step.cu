@@ -154,9 +154,6 @@ int dm_step_layout(int nl, int n, int chain_len, int maxrows, int W, StepLayout*
 }
 int dm_step_smem_bytes(const StepLayout& L, int tiles) { return (L.hot_floats + L.env_floats * tiles) * static_cast<int>(sizeof(float)); }
 
-#ifndef DM_PGS_BLOCK
-#define DM_PGS_BLOCK 2   // solver steps evaluated per block of the projected Gauss-Seidel sweeps (measured on a B200: 1 -> 1.22 M, 2 -> 1.49 M, 4 -> 1.32 M, 8 -> 0.95 M policy steps/s)
-#endif
 // Projected Gauss-Seidel in impulse space, 10 sweeps in btMultiBodyConstraintSolver::solveSingleIteration's row order (joint limits in
 // alternating order, contact normals, friction pairs).  Lanes = rows for the state that is wide: every lane keeps w = (A lambda)_row of ITS rows in
 // registers (S rows per lane: row = lane + s W).  The sequential part is evaluated in blocks of B consecutive solver steps of one section:
@@ -313,7 +310,7 @@ __device__ __noinline__ void solve_rows(int NL, int P, float* mani, int alive, u
     const int NR = NL + 3 * P;
     const int NRmax = (W == 32) ? NR : wmax(NR);
     const int nslots = (NRmax + W - 1) / W;
-    constexpr int kPgsBlock = DM_PGS_BLOCK;
+    constexpr int kPgsBlock = 2;   // solver steps evaluated per block of the projected Gauss-Seidel sweeps (measured on a B200: 1 -> 1.22 M, 2 -> 1.49 M, 4 -> 1.32 M, 8 -> 0.95 M policy steps/s)
     constexpr int kSlots = 2;   // rows per lane in the general path: the host caps the row capacity at dm_step_y_stride(W) (32 humanoid3d, 52 dog3d)
 #pragma unroll
     for (int s = 0; s < kSlots; ++s) {
@@ -1120,7 +1117,7 @@ __device__ __noinline__ void vel_pass(float jvx, float jvy, float jvz, bool want
 //   bit 1 (kVarRootRot) --sync_char_root_rot: the heading sync of cSceneImitate::SyncKinCharNewCycle at a clip wrap
 template <int W, bool DEBUG, int VAR>
 __global__ void __launch_bounds__(kStepMaxThreads, 1) dm_step_kernel(const DevModel* __restrict__ gm, DevState st, const double* __restrict__ frame_times,
-                                                                       const float* __restrict__ frames, double dt, int n_updates, int sim_substeps, StepLayout LY, int sync_mode) {
+                                                                       const float* __restrict__ frames, double dt, int n_updates, int sim_substeps, StepLayout LY) {
     constexpr bool TASK = (VAR & kVarTask) != 0, ROOTROT = (VAR & kVarRootRot) != 0;
     using T = Tl<W>;
     extern __shared__ __align__(16) float sm[];
@@ -1284,7 +1281,6 @@ __global__ void __launch_bounds__(kStepMaxThreads, 1) dm_step_kernel(const DevMo
     int mcnt = 4;   // cached points of this lane's link after the last collision pass; unknown at the start of a launch: forces the first read
     const int stages_per_upd = sim_substeps + 1;
     const int total_stages = n_updates * stages_per_upd;
-    const int sync_period = sync_mode > 0 ? 1 : (sync_mode == 0 ? stages_per_upd : (sync_mode <= -1000 ? 0 : -sync_mode * stages_per_upd));
 #pragma unroll 1
     for (int stage = 0; stage <= total_stages; ++stage) {
         // the manifold of this lane's link is read by the collision pass of a Bullet sub-step: start pulling its two cache lines in now
@@ -1384,7 +1380,9 @@ __global__ void __launch_bounds__(kStepMaxThreads, 1) dm_step_kernel(const DevMo
         }
         PROF(1);
         if (stage == total_stages) break;
-        if (sync_period != 0 && (stage % sync_period) == 0) { if (__syncthreads_and(!alive)) break; }
+        // block barrier after every stage (Stable-PD stage, each Bullet sub-step): measured on a B200, 2.12 M vs 2.11 M policy steps/s with one per update,
+        // 1.94 / 1.89 / 1.78 M with one every 2 / 4 updates / none (warps that drift apart thrash the instruction cache)
+        if (__syncthreads_and(!alive)) break;
         PROF(2);
         if (__ballot_sync(0xffffffffu, alive) == 0u) continue;   // both environments of this warp are frozen
         const int ph = stage % stages_per_upd;      // 0: Stable-PD stage, 1..sim_substeps: Bullet sub-steps
@@ -1593,15 +1591,15 @@ __global__ void __launch_bounds__(kStepMaxThreads, 1) dm_step_kernel(const DevMo
 }
 
 // explicit instantiations used by capi.cu: (tile width, debug dumps)
-template __global__ void dm_step_kernel<16, false, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
-template __global__ void dm_step_kernel<32, false, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
-template __global__ void dm_step_kernel<16, true, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
-template __global__ void dm_step_kernel<32, true, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
+template __global__ void dm_step_kernel<16, false, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
+template __global__ void dm_step_kernel<32, false, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
+template __global__ void dm_step_kernel<16, true, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
+template __global__ void dm_step_kernel<32, true, 0>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
 // AMP task scenes (target_amp / heading_amp): same step with the task block advanced after every update
-template __global__ void dm_step_kernel<16, false, kVarTask>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
-template __global__ void dm_step_kernel<32, false, kVarTask>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
+template __global__ void dm_step_kernel<16, false, kVarTask>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
+template __global__ void dm_step_kernel<32, false, kVarTask>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
 // --sync_char_root_rot true (dog3d_spin)
-template __global__ void dm_step_kernel<16, false, kVarRootRot>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
-template __global__ void dm_step_kernel<32, false, kVarRootRot>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout, int);
+template __global__ void dm_step_kernel<16, false, kVarRootRot>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
+template __global__ void dm_step_kernel<32, false, kVarRootRot>(const DevModel*, DevState, const double*, const float*, double, int, int, StepLayout);
 
 }  // namespace dmk

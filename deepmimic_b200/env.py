@@ -250,10 +250,10 @@ class DeepMimicBatchEnv:
 
     def check_solver_capacity(self, raise_on_overflow=True):
         """Call at reset / collect boundaries (host synchronisation).  Raises (or warns) when any environment exceeded the solver's row
-        capacity since the handle was created: raise DM_MAX_ROWS or treat the affected episodes as invalid."""
+        capacity since the handle was created.  The capacity is fixed per character (DESIGN.md 5.5): treat the affected episodes as invalid."""
         over = self._core.counters()[1]
         if over:
-            msg = "deepmimic_b200: %d environment(s) exceeded the contact-solver row capacity; contacts were truncated (set DM_MAX_ROWS higher)" % over
+            msg = "deepmimic_b200: %d environment(s) exceeded the contact-solver row capacity; contacts were truncated, so their episodes are invalid" % over
             if raise_on_overflow:
                 raise RuntimeError(msg)
             import warnings

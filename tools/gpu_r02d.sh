@@ -4,4 +4,3 @@ timeout 300 python tools/diag_target.py 2>&1 | tail -80
 DM_LIB=$PWD/deepmimic_b200/libdeepmimic_b200_prof.so timeout 300 python tools/section_profile.py 2>&1 | tail -40
 timeout 900 python -m pytest tests/test_qd_envelope_gpu.py tests/test_parity2_gpu.py -m gpu -q --tb=short -s 2>&1 | tail -60
 DM_LIB=$PWD/deepmimic_b200/libdeepmimic_b200_precise.so timeout 600 python -m pytest tests/test_qd_envelope_gpu.py -m gpu -q --tb=short -s 2>&1 | tail -30
-for m in 1 -2; do DM_SYNC_EVERY_STAGE=$m timeout 300 python bench.py --steps 128 --no-cpu-baseline 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('SYNC_MODE $m', d['value'], d['roofline']['kernel_ms'])"; done
